@@ -252,6 +252,27 @@ def run_reference(args):
     print(json.dumps(line))
 
 
+DUMP_BYTES = 60 * 10**6  # keeps --dump-outputs under 64 MB with the .npy headers
+
+
+def dump_outputs(d, flags, scores, n_candidates):
+    """DIR/<name>.npy of one step's results. When all rows would exceed DUMP_BYTES, a fixed, seeded sample of the rows
+    (samples) is written; sample_rows lists them."""
+    # pose_scores is NaN where no image was classified (include/gpd_b200.h): those NaNs, at poses pose_flags marks as not
+    # classified, are written as 0. Every other score is written as computed, so a value the contract does not allow shows.
+    classified = (flags & 3) == 3  # GPDB_POSE_VALID | GPDB_POSE_FILTERED
+    scores = np.where(~classified & np.isnan(scores), np.float32(0), scores)
+    n, P = flags.shape
+    per_row = 2 * 4 * P + 8  # flags and scores as float32, the row number as float64
+    rows = np.arange(n)
+    if n * per_row > DUMP_BYTES:
+        rows = np.sort(np.random.default_rng(0).choice(n, DUMP_BYTES // per_row, replace=False))
+    os.makedirs(d, exist_ok=True)
+    for name, a in (("pose_flags", flags[rows].astype(np.float32)), ("pose_scores", scores[rows].astype(np.float32)),
+                    ("sample_rows", rows.astype(np.float64)), ("n_candidates", np.array([n_candidates], np.float64))):
+        np.save(os.path.join(d, name + ".npy"), a)
+
+
 def _divert_stdout():
     """Send everything written to file descriptor 1 (Python AND native libraries: NCCL prints its version banner to
     stdout when NCCL_DEBUG >= VERSION) to stderr; the ONE JSON line is printed after _restore_stdout."""
@@ -282,7 +303,15 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--lenet-impl", type=int, default=0)
     ap.add_argument("--no-preprocess", action="store_true", help="skip the secondary gpdb_preprocess measurement")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed to DIR/<name>.npy (pose_flags, pose_scores [samples, poses] "
+                         "as float32; the library's NaN score of a pose with no classified image is written as 0; "
+                         "sample_rows, n_candidates), to compare two builds output for output")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the device path's results; --impl reference has none")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -347,6 +376,20 @@ def main():
             return ctx.detect_sharded_resident(d_sidx.data_ptr(), n, slot_samples, d_gath.data_ptr(), stats)
         return ctx.detect_resident(d_sidx.data_ptr(), n, d_flags.data_ptr(), d_scores.data_ptr(), stats)
 
+    def last_step_outputs():
+        """(pose_flags, pose_scores) [n_all, P] as the caller of step_resident receives them; N > 1: decoded from the
+        all-gathered slots (include/gpd_b200.h: [scores f32 slot_samples*P][flags u8 slot_samples*P, padded])."""
+        if world == 1:
+            return d_flags.view(n, P).cpu().numpy(), d_scores.view(n, P).cpu().numpy()
+        g = d_gath.cpu().numpy()
+        flags, scores = [], []
+        for r in range(world):
+            lo_r, hi_r, _ = lib.shard_bounds(n_all, r, world)
+            s = g[r * slot_b:(r + 1) * slot_b]
+            scores.append(s[:4 * slot_samples * P].view(np.float32)[:(hi_r - lo_r) * P])
+            flags.append(s[4 * slot_samples * P:][:(hi_r - lo_r) * P])
+        return np.concatenate(flags).reshape(n_all, P), np.concatenate(scores).reshape(n_all, P)
+
     for _ in range(args.warmup):
         step_resident()
     torch.cuda.synchronize()
@@ -370,6 +413,8 @@ def main():
     if world > 1:
         dist.barrier()
     clocks = sampler.stop()
+    # the last timed step's results, copied before the serial passes below overwrite the buffers
+    outputs = last_step_outputs() if args.dump_outputs and rank == 0 else None
     # per-stage device times from a SERIAL pass (outside the timed region): in the timed steps the hand search of the chunks
     # ahead runs concurrently with images / LeNet of the current chunk, so its stage timers overlap the others
     ctx.set_overlap(0)
@@ -469,6 +514,8 @@ def main():
                       "call": "gpdb_detect_select (detectGrasps + selectGrasps, top-100 picked on the device)"}
 
     if rank == 0:
+        if outputs is not None:
+            dump_outputs(args.dump_outputs, *outputs, ncand_all)
         st = stage_ms / args.steps  # per step, this rank
         peaks = {}
         try:

@@ -1,8 +1,8 @@
 """Weight import from the reference's other backends' formats (SURVEY.md 8(f).2): `.caffemodel` (Caffe backend) and
 OpenVINO IR `.xml` + `.bin` -> the .bin parameter-directory layout (gpdb_read_weights_file / gpdb_load_weights_file).
 
-CPU: the wire-level parsers against files written by this test (a minimal protobuf encoder / an IR skeleton) and — in
-the build container, where /root/reference exists — against the reference's own model files, which must reproduce the
+CPU: the wire-level parsers against files written by this test (a minimal protobuf encoder / an IR skeleton) and against
+the reference's own model files, rebuilt byte for byte from tests/golden/ref_model_files.npz, which must reproduce the
 shipped .bin parameters bit for bit. GPU: a context loaded from a .caffemodel scores like one given the arrays."""
 import os
 import struct
@@ -12,9 +12,7 @@ import pytest
 
 from conftest import load_weights
 from gpd_b200 import lib
-
-REF = "/root/reference/models"
-NAMES = ["conv1_weights", "conv1_biases", "conv2_weights", "conv2_biases", "ip1_weights", "ip1_biases", "ip2_weights", "ip2_biases"]
+from oracle.reference_data import rebuild_model_file
 
 
 def _varint(v):
@@ -104,15 +102,16 @@ def test_openvino_ir_parser(tmp_path):
             assert np.array_equal(a, e)
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="the reference's model files exist only in the build container")
-def test_reference_model_files_reproduce_the_bin_parameters():
-    for ch, path in ((15, f"{REF}/caffe/15channels/two_views_15_channels_90_deg_no_flipping.caffemodel"),
-                     (3, f"{REF}/caffe/3channels/bottles_boxes_cans_5xNeg.caffemodel")):
-        arrs, _ = lib.read_weights_file(path, ch)
-        ref = [np.fromfile(f"{REF}/lenet/{ch}channels/params/{n}.bin", dtype=np.float32) for n in NAMES]
-        assert all(np.array_equal(a, r) for a, r in zip(arrs, ref)), ch
-    arrs, relu = lib.read_weights_file(f"{REF}/openvino/two_views_12_channels_curv_axis.bin", 12)
+def test_reference_model_files_reproduce_the_bin_parameters(tmp_path, golden_dir):
+    """The .caffemodel files of the 15- and 3-channel nets give the reference's .bin parameters (gpd_b200/weights/, equal to
+    models/lenet/<ch>channels/params/), the OpenVINO IR of the 12-channel net its ReLU net."""
+    g = np.load(os.path.join(golden_dir, "ref_model_files.npz"))
+    for ch in (15, 3):
+        ref, _ = load_weights(ch)
+        arrs, _ = lib.read_weights_file(rebuild_model_file(g, ch, ref, tmp_path), ch)
+        assert all(np.array_equal(a, np.ravel(r)) for a, r in zip(arrs, ref)), ch
     w12, _ = load_weights(12)
+    arrs, relu = lib.read_weights_file(rebuild_model_file(g, 12, w12, tmp_path), 12)
     assert relu == 3 and all(np.array_equal(a, np.ravel(r)) for a, r in zip(arrs, w12))
 
 

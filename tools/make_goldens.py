@@ -12,9 +12,17 @@ independent ground truth the reference itself links against). The GPU box never 
   gpd_b200/weights/lenet_{15,3,12}ch.npz  the reference weights in the .bin layout
   tests/golden/krylon_preprocess.npz      raw tutorials/krylon.pcd points + the oracle's preprocessing outputs
                                           + an independent float64 PCA normal per point (`--only preprocess`)
+  tests/golden/cfg/*.cfg                  the reference's cfg files the parser tests read, and
+  tests/golden/ref_config_parser.json     what the reference's own cfg parser (oracle/_ref) answers on them (`--only ref_config`)
+  tests/golden/ref_model_files.npz        the reference's .caffemodel / IR files of the shipped nets without their weight
+                                          payloads, which tests rebuild from gpd_b200/weights/ (`--only ref_models`)
 """
+import hashlib
+import json
 import os
 import re
+import shutil
+import subprocess
 import sys
 import tempfile
 import zlib
@@ -181,14 +189,67 @@ def krylon_preprocess():
     print("krylon_preprocess:", len(raw), "->", len(P))
 
 
+def ref_config():
+    """The cfg files of the parser tests (oracle/reference_data.py), and the answers of the reference's own util::ConfigFile /
+    HandGeometry / ImageGeometry (oracle/_ref, built from the reference's sources) on them."""
+    import ctypes
+    from oracle import reference_data as t
+    cfg = os.path.join(G, "cfg")
+    os.makedirs(cfg, exist_ok=True)
+    for name in sorted(set(t.SHIPPED_CFGS + t.GEOMETRY_CFGS + ("vino_params_12channels.cfg", "all_axes_vino_12channels.cfg",
+                                                                "image_geometry_12channels.cfg"))):
+        shutil.copyfile(f"{REF}/cfg/{name}", os.path.join(cfg, name))
+    subprocess.check_call(["make", "-C", os.path.join(ROOT, "oracle"), "_ref", f"REF={REF}", "-s"])
+    R = ctypes.CDLL(os.path.join(ROOT, "oracle", "_ref", "libgpd_ref_config.so"))
+    with tempfile.TemporaryDirectory() as d:
+        ans = t.config_parser_answers(R, True, cfg, d)
+    with open(os.path.join(G, "ref_config_parser.json"), "w") as f:
+        json.dump(ans, f, indent=0, sort_keys=True)
+    print("ref_config_parser:", len(ans), "answers")
+
+
+def ref_models():
+    """Each model file of oracle/reference_data.MODEL_FILES as a skeleton (the file with its eight weight payloads cut out), the
+    payloads' offsets, the file's SHA-256 and, for the IR, its .xml. The payloads are the committed weights in the blob
+    layout, which this checks against the reference's .bin parameters."""
+    from oracle.reference_data import MODEL_FILES, blob_layout
+    out = {}
+    for ch, name in MODEL_FILES.items():
+        ir = name.endswith(".bin")
+        raw = open(f"{REF}/models/{'openvino' if ir else f'caffe/{ch}channels'}/{name}", "rb").read()
+        z = np.load(os.path.join(W, f"lenet_{ch}ch.npz"))
+        w = [z[n] for n in NAMES]
+        if not ir:
+            ref = scenes.load_weights_dir(f"{REF}/models/lenet/{ch}channels/params/")
+            assert all(np.array_equal(np.ravel(a), r) for a, r in zip(w, ref)), ch
+        skel, cuts, pos = bytearray(), [], 0
+        for k, b in enumerate(blob_layout(w)):
+            off = raw.find(b.tobytes(), pos)
+            assert off >= 0, (name, NAMES[k])
+            skel += raw[pos:off]
+            cuts.append((off, k, b.nbytes))
+            pos = off + b.nbytes
+        skel += raw[pos:]
+        out[f"{ch}_skeleton"] = np.frombuffer(bytes(skel), np.uint8)
+        out[f"{ch}_cuts"] = np.array(cuts, np.int64)
+        out[f"{ch}_sha256"] = np.array(hashlib.sha256(raw).hexdigest())
+        if ir:
+            out[f"{ch}_xml"] = np.frombuffer(open(f"{REF}/models/openvino/{name[:-4]}.xml", "rb").read(), np.uint8)
+        print(f"{name}: {len(raw)} bytes -> {len(skel)} byte skeleton")
+    np.savez_compressed(os.path.join(G, "ref_model_files.npz"), **out)
+
+
 if __name__ == "__main__":
     os.makedirs(G, exist_ok=True)
     os.makedirs(W, exist_ok=True)
-    if "--only" in sys.argv and sys.argv[sys.argv.index("--only") + 1] == "preprocess":
-        krylon_preprocess()
+    only = {"preprocess": krylon_preprocess, "ref_config": ref_config, "ref_models": ref_models}
+    if "--only" in sys.argv:
+        only[sys.argv[sys.argv.index("--only") + 1]]()
         sys.exit(0)
     krylon_oracle()
     cv_pins()
     lenet_caffe(15)
     lenet_caffe(3)
     lenet_ir_12ch()
+    ref_config()
+    ref_models()
