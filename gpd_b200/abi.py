@@ -145,6 +145,44 @@ def default_preprocess_params(**over):
     return p
 
 
+class PlaneParams(C.Structure):
+    """gpdb_plane_params — the support-plane fit of sample_above_plane (include/gpd_b200_plane.h)."""
+
+    _fields_ = [
+        ("distance_threshold", C.c_double),
+        ("num_hypotheses", C.c_int32),
+        ("seed", C.c_uint64),
+    ]
+
+
+class PlaneInfo(C.Structure):
+    """gpdb_plane_info — what the plane fit found."""
+
+    _fields_ = [
+        ("coefficients", C.c_float * 4),
+        ("hypothesis_coefficients", C.c_float * 4),
+        ("hypothesis", C.c_int32),
+        ("hypothesis_inliers", C.c_int32),
+        ("inliers", C.c_int32),
+        ("refined", C.c_int32),
+    ]
+
+
+def default_plane_params(**over):
+    """Defaults of gpdb_plane_params_default: threshold 0.01 (cloud.cpp:418), 1024 hypotheses, seed 1."""
+    p = PlaneParams(0.01, 1024, 1)
+    for k, v in over.items():
+        setattr(p, k, v)
+    return p
+
+
+def plane_info_to_dict(info):
+    return {"coefficients": np.array(info.coefficients[:], np.float32),
+            "hypothesis_coefficients": np.array(info.hypothesis_coefficients[:], np.float32),
+            "hypothesis": info.hypothesis, "hypothesis_inliers": info.hypothesis_inliers, "inliers": info.inliers,
+            "refined": info.refined}
+
+
 def default_params(channels=15, **over):
     """The reference defaults (gpdb_params_default in C), restated for the oracle loader.
 

@@ -24,6 +24,7 @@ EXPORTS = [
     "gpdb_get_cloud", "gpdb_get_cloud_source_index", "gpdb_preprocess_timings", "gpdb_detect_select", "gpdb_load_weights_file", "gpdb_read_weights_file", "gpdb_set_samples",
     "gpdb_comm_unique_id", "gpdb_comm_init", "gpdb_comm_destroy", "gpdb_shard_bounds", "gpdb_set_cloud_bcast",
     "gpdb_detect_sharded", "gpdb_detect_sharded_resident", "gpdb_slot_bytes", "gpdb_find_clusters", "gpdb_reevaluate", "gpdb_set_overlap",
+    "gpdb_plane_params_default", "gpdb_sample_above_plane",
 ]
 
 
@@ -84,6 +85,9 @@ def lib():
     L.gpdb_find_clusters.argtypes = [vp, vp, C.c_int32, C.c_int32, vp]
     L.gpdb_reevaluate.argtypes = [vp, vp, C.c_int32, vp]
     L.gpdb_set_overlap.argtypes = [vp, C.c_int32]
+    L.gpdb_plane_params_default.argtypes = [C.POINTER(abi.PlaneParams)]
+    L.gpdb_plane_params_default.restype = None
+    L.gpdb_sample_above_plane.argtypes = [vp, C.POINTER(abi.PlaneParams), vp, C.POINTER(abi.PlaneInfo)]
     _LIB = L
     return L
 
@@ -124,6 +128,15 @@ def preprocess_params(**over):
             p.workspace[:] = list(v)
         else:
             setattr(p, k, v)
+    return p
+
+
+def plane_params(**over):
+    """gpdb_plane_params with the library defaults (threshold 0.01, 1024 hypotheses, seed 1), overridden by keyword."""
+    p = abi.PlaneParams()
+    lib().gpdb_plane_params_default(C.byref(p))
+    for k, v in over.items():
+        setattr(p, k, v)
     return p
 
 
@@ -211,6 +224,17 @@ class Context:
         else:
             out["src"] = np.zeros(0, np.int32)
         return out
+
+    def sample_above_plane(self, pp=None):
+        """Cloud::sampleAbovePlane on the installed cloud (gpdb_sample_above_plane): (off-plane indices ascending, info
+        dict). An empty index array means the plane fit failed and the whole cloud stays sampled."""
+        if pp is None:
+            pp = plane_params()
+        n_pts = self._check(lib().gpdb_get_cloud(self.h, None, None, None))
+        idx = np.zeros(max(n_pts, 1), np.int32)
+        info = abi.PlaneInfo()
+        n = self._check(lib().gpdb_sample_above_plane(self.h, C.byref(pp), _p(idx), C.byref(info)))
+        return idx[:n].copy(), abi.plane_info_to_dict(info)
 
     # ---- multi-GPU sharding inside the boundary (gpdb_comm_*, SURVEY.md 8(e)) ----
     def comm_init(self, unique_id, rank, nranks):

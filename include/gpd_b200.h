@@ -269,8 +269,9 @@ void gpdb_preprocess_params_default(gpdb_preprocess_params *p);
  * on the device, and installs the processed cloud in the context exactly as gpdb_set_cloud would (the neighbour
  * grid is built from the device copy). Inputs as gpdb_set_cloud (raw cloud, n_points may be millions); `normals`
  * may be NULL when estimate_normals = 1. Returns the number of processed points N' (>= 0) or a negative error.
- * Not covered: refine_normals_k, remove_outliers, sample_above_plane (PCL filters outside the default cfg) and
- * Cloud::subsample (host-side RNG; the sample indices are an input of gpdb_detect).
+ * Not covered: refine_normals_k, remove_outliers (PCL filters outside the default cfg), sample_above_plane (a separate
+ * call on the installed cloud: gpdb_sample_above_plane) and Cloud::subsample (host-side RNG; the sample indices are an
+ * input of gpdb_detect).
  * Semantics that differ from the reference by specification (DESIGN.md "preprocessing"): the voxel set is an
  * exact set (the reference's std::set comparator is not a strict weak order), output order = descending index
  * of each voxel's first point (the reference's iteration order whenever its de-duplication succeeds). */
@@ -291,6 +292,36 @@ int gpdb_get_cloud_source_index(gpdb_ctx *ctx, int32_t *src_out);
 /* Device time (ms, CUDA events) of the stages of the last gpdb_preprocess call:
  * ms[0] upload, ms[1] NaN/workspace filter, ms[2] voxelise, ms[3] grid build, ms[4] normals, ms[5] whole call. */
 int gpdb_preprocess_timings(const gpdb_ctx *ctx, double ms_out[6]);
+
+/* Parameters of the support-plane fit (include/gpd_b200_plane.h). */
+typedef struct gpdb_plane_params {
+  double distance_threshold; /* inlier distance (cloud.cpp:418: 0.01)                                          */
+  int32_t num_hypotheses;    /* RANSAC triples evaluated, 1 .. GPDB_PLANE_MAX_HYPOTHESES (default 1024)         */
+  uint64_t seed;             /* seed of the counter-based draw of the triples                                    */
+} gpdb_plane_params;
+
+/* Defaults: threshold 0.01, 1024 hypotheses, seed 1. */
+void gpdb_plane_params_default(gpdb_plane_params *pp);
+
+/* What the fit found (all zero and hypothesis = -1 when no triple was valid). */
+typedef struct gpdb_plane_info {
+  float coefficients[4];            /* final plane a, b, c, d: refined, or the winner's when not refined           */
+  float hypothesis_coefficients[4]; /* plane of the winning triple                                                 */
+  int32_t hypothesis;               /* winning hypothesis h, -1 when none is valid                                  */
+  int32_t hypothesis_inliers;       /* its inlier count                                                            */
+  int32_t inliers;                  /* inliers of the final plane                                                  */
+  int32_t refined;                  /* 1 when the coefficients were refined (the winner has >= 4 inliers)          */
+} gpdb_plane_info;
+
+/* Replaces: Cloud::sampleAbovePlane (cloud.cpp:407-435; cfg key sample_above_plane, candidates_generator.cpp:32-34):
+ * PCL SACSegmentation (RANSAC plane, optimizeCoefficients) + ExtractIndices(negative) on the device, over the cloud
+ * installed by gpdb_preprocess or gpdb_set_cloud, as the deterministic variant specified in include/gpd_b200_plane.h.
+ * off_plane_idx_out (room for N) receives the indices of the points off the fitted plane in ascending order; these are
+ * the cloud's sample indices that Cloud::subsample then draws from. Returns their number; 0 = the plane fit failed (fewer
+ * than 3 points, every triple degenerate, or no point / every point on the plane: the caller keeps the whole cloud);
+ * negative = error (no cloud, bad parameters). info_out may be NULL. */
+int gpdb_sample_above_plane(gpdb_ctx *ctx, const gpdb_plane_params *pp, int32_t *off_plane_idx_out,
+                            gpdb_plane_info *info_out);
 
 /* Replaces: HandSearch::reevaluateHypotheses (hand_search.cpp:66-134; GraspDetector::evalGroundTruth,
  * grasp_detector.cpp:523-527): the given hands (sample, frame, top, finger_idx are read) are re-labelled against the cloud
